@@ -9,6 +9,7 @@ one frame (+ its 8 IMU samples) for every sequence on every GPU.
 
   python bench.py --gpus N --steps K --warmup W              # this repo (CUDA)
   python bench.py --impl reference --gpus N --steps K --warmup W   # reference CPU arithmetic, all host cores
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # + every sequence's state after the last step, DIR/<name>.npy
 
 Prints ONE JSON line (rank 0).  `value` = frames/s with the frames already resident in HBM;
 `e2e` = the same through the estimator-level C ABI with pinned HOST frames (H2D inside the timed
@@ -374,6 +375,33 @@ def build_roofline(prof, K, peaks, seqs_per_launch, pass_ms):
     return roofline, host_phases
 
 
+DUMP_P_SEQS = 32  # covariances in a --dump-outputs directory: a fixed sample of sequences keeps it far below 64 MB at every config
+
+
+def dump_outputs(out_dir, bts, sizes):
+    """Writes what a caller of xivo_batch_step holds after the last step, for every sequence of this GPU in sequence order, as
+    out_dir/<name>.npy (float64): the pose gsb, velocity, IMU biases and gravity rotation, the estimator counters, the tracked features
+    (ids and pixel positions padded with -1: every value is finite) and the full error-state covariance of a seeded sample of the sequences."""
+    seqs = [(b, s) for b, n in zip(bts, sizes) for s in range(n)]
+    out = dict(gsb=np.stack([b.gsb(s) for b, s in seqs]))
+    motion = [b.motion(s) for b, s in seqs]
+    for i, name in enumerate(("vsb", "bg", "ba", "Rsg")):
+        out[name] = np.stack([m[i] for m in motion])
+    out["counters"] = np.array([list(b.counters(s).values()) for b, s in seqs], dtype=np.float64)
+    tracked = [b.tracked_features(s)[:2] for b, s in seqs]
+    width = max([len(ids) for ids, _ in tracked] + [1])
+    out["tracked_ids"], out["tracked_xy"] = np.full((len(seqs), width), -1.0), np.full((len(seqs), width, 2), -1.0)
+    for i, (ids, xy) in enumerate(tracked):
+        out["tracked_ids"][i, : len(ids)], out["tracked_xy"][i, : len(ids)] = ids, xy
+    pick = np.sort(np.random.default_rng(0).choice(len(seqs), min(DUMP_P_SEQS, len(seqs)), replace=False))
+    out["P_sample_seqs"] = pick.astype(np.float64)
+    out["P_sample"] = np.stack([seqs[i][0].P(seqs[i][1]) for i in pick])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {name: a.shape for name, a in out.items()}
+
+
 def run_ours(args):
     # host CPUs: the library's worker pool (workpool.h) is shared by the NB batches of this process; each batch
     # also has one driver thread (the Python thread inside xivo_batch_step), so workers + drivers = CPU budget
@@ -560,6 +588,8 @@ def run_ours(args):
     log("e2e pass", r_e2e["ms"], "ms")
     r_prof = timed(not args.profile_e2e, args.profile_level, K_prof)
     log("profiled pass", r_prof["ms"], "ms")
+    if args.dump_outputs and rank == 0:
+        log("outputs written to", args.dump_outputs, dump_outputs(args.dump_outputs, bts, sizes))
     frames_total = world * B * K * FPS
     value = frames_total / (r_dev["ms"] * 1e-3)
     e2e = frames_total / (r_e2e["ms"] * 1e-3)
@@ -679,7 +709,12 @@ def main():
     ap.add_argument("--no-numa", dest="numa", action="store_false", help="leave the process on every allowed CPU instead of the NUMA node of its GPU")
     ap.add_argument("--prefetch", action="store_true", help="e2e pass with xivo_batch_prefetch_frames (the upload of frame k + 1 is started before frame k is processed); measured neutral on the B200 box (profiles/r02z_sweep.txt), so the default is the plain call")
     ap.add_argument("--ingest", default="auto", choices=["auto"] + list(INGEST_MODES), help="how pinned host frames reach the device (e2e pass); auto = calibrate both before the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed passes, write the state every sequence of GPU 0 holds after its last step "
+                                                          "(pose, motion, counters, tracked features, a seeded sample of covariances) as DIR/<name>.npy; "
+                                                          "the inputs depend only on the arguments, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of this repository's path (--impl ours)")
     if args.warmup < 3:
         args.warmup = 3
     c = select_config(args.config)

@@ -17,8 +17,9 @@ out = {}
 with tempfile.TemporaryDirectory() as td:
     for name, G, F, duration, seed, sim_depths, over, offset in CASES:
         d = ref_runner.run_subprocess(CFG, G, F, duration, seed, sim_depths, os.path.join(td, name + ".npz"), overrides=over, pc_offset_ns=offset)
-        for k in ("gsb", "ts", "n_instate", "gauge", "ids", "P"):
+        for k in ("gsb", "ts", "n_instate", "gauge", "ids"):
             out[f"{name}.{k}"] = d[k]
+        out[f"{name}.P_upper"] = d["P"][np.triu_indices(len(d["P"]))]  # symmetric to 1e-19 (test_reference_pin.sym_from_upper)
         if name in ("small_89", "default_203"):  # the reference's read-back accessors at the end of the run (boundary-parity fixtures)
             for k in d.files:
                 if k.startswith("acc."):

@@ -156,6 +156,55 @@ def test_stream_tables_never_hand_one_frame_to_two_sequences_at_the_default_size
         assert len(np.unique(key[f])) == n, f
 
 
+def test_dump_outputs_writes_every_sequence_in_order(tmp_path):
+    """--dump-outputs with stand-in batches (the read-back methods of xivo_b200.pyxivo.Batch): one row per sequence in sequence order
+    across batches, finite float arrays only, tracked features padded, the covariance sample seeded, and below 64 MB at every config's default size."""
+    import numpy as np
+
+    class FakeBatch:
+        def __init__(self, first, N):
+            self.first, self.N = first, N
+
+        def gsb(self, s):
+            return np.full((3, 4), float(self.first + s))
+
+        def motion(self, s):
+            k = float(self.first + s)
+            return np.full(3, k), np.full(3, k + 0.1), np.full(3, k + 0.2), np.full((3, 3), k + 0.3)
+
+        def counters(self, s):
+            return dict(a=self.first + s, b=7)
+
+        def tracked_features(self, s):
+            n = (self.first + s) % 4
+            return np.arange(n, dtype=np.int32) + 100, np.full((n, 2), 0.5), np.ones(n, np.int32)
+
+        def P(self, s):
+            return np.full((self.N, self.N), float(self.first + s))
+
+    sizes = [30, 20, 20]
+    bts = [FakeBatch(0, 5), FakeBatch(30, 5), FakeBatch(50, 5)]
+    shapes = bench.dump_outputs(str(tmp_path / "a"), bts, sizes)
+    bench.dump_outputs(str(tmp_path / "b"), bts, sizes)
+    d = {name: np.load(str(tmp_path / "a" / (name + ".npy"))) for name in shapes}
+    assert all(a.dtype == np.float64 and np.isfinite(a).all() for a in d.values())
+    assert np.array_equal(d["gsb"][:, 0, 0], np.arange(70)) and np.array_equal(d["Rsg"][:, 2, 2], np.arange(70) + 0.3)
+    assert np.array_equal(d["counters"], np.stack([np.arange(70), np.full(70, 7)], 1))
+    assert d["tracked_ids"].shape == (70, 3) and d["tracked_ids"][5].tolist() == [100, -1, -1] and (d["tracked_xy"][5, 1:] == -1).all()
+    pick = d["P_sample_seqs"].astype(int)
+    assert len(pick) == bench.DUMP_P_SEQS and np.array_equal(d["P_sample"][:, 0, 0], pick)
+    for name in shapes:  # the same arguments give the same files
+        assert np.array_equal(d[name], np.load(str(tmp_path / "b" / (name + ".npy"))))
+    try:  # every config at its default size: sequences x (pose, motion, counters, tracked features) + the covariance sample
+        for n, c in bench.CONFIGS.items():
+            bench.select_config(n)
+            tracked = bench.load_cfg()["tracker_cfg"]["num_features_max"]
+            N = 23 + 6 * c["G"] + 3 * c["F"]
+            assert c["seqs"] * (12 + 18 + 12 + 3 * tracked) * 8 + bench.DUMP_P_SEQS * N * N * 8 < 64 << 20, n
+    finally:
+        bench.select_config(1)
+
+
 def test_cpulist_parser_and_numa_placement_is_optional():
     import bench
 

@@ -402,7 +402,8 @@ def test_homography_mask_matches_the_oracle_and_cv2(hh, method):
     assert flips <= 2, f"{flips} mask entries differ over 48 scenes"
 
 
-REFERENCE_CFG = "/root/reference/cfg"
+# the configs shipped in the reference's cfg/ directory, parsed (tests/golden/make_golden_cfgs.py)
+REFERENCE_CFGS = os.path.join(ROOT, "tests", "golden", "reference_cfgs.json")
 # what each estimator / tracker config shipped with the reference does when it is handed to the host parser unmodified
 # (None = accepted; otherwise a fragment of the refusal).  DESIGN.md §8 discusses every entry.
 SHIPPED = {
@@ -417,15 +418,10 @@ SHIPPED = {
 }
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE_CFG), reason="the reference checkout is only present in the authoring container")
 @pytest.mark.parametrize("name,refusal", sorted(SHIPPED.items()))
 def test_shipped_reference_configs_through_the_host_parser(hh, name, refusal):
-    cwd = os.getcwd()
-    os.chdir(os.path.dirname(REFERENCE_CFG))  # camera_cfg / tracker_cfg may be relative paths
-    try:
-        cfg = sim.load_cfg(os.path.join("cfg", name))
-    finally:
-        os.chdir(cwd)
+    with open(REFERENCE_CFGS) as f:
+        cfg = json.load(f)[name]
     h = hh.hh_create(json.dumps(cfg).encode(), 15, 30, int("tracker_only" in name))
     if refusal is None:
         assert h, hh.hh_error()
